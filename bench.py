@@ -304,7 +304,11 @@ def main():
     ap.add_argument("--dense-n", type=int, default=2000, help="n of the exact-GP measurement (BASELINE configs[0]; 0 = skip; --impl reference times it too)")
     ap.add_argument("--laplace-n", type=int, default=1000000, help="n of the Laplace-Vecchia (bernoulli_logit) measurement, BASELINE configs[4] (0 = skip)")
     ap.add_argument("--laplace-ref-n", type=int, default=100000, help="--impl reference: n of the Laplace-Vecchia evaluation sub-problem (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed steps computed in their last step to DIR/<name>.npy (float64), for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -424,6 +428,10 @@ def main():
         chk(lib.gpbdev_vecchia_timer_stop(eng, C.byref(ms)))
         kernel_ms.append(ms.value)
     barrier()
+    outputs = {}  # --dump-outputs: name -> array of the last timed step
+    sums = np.zeros(9)
+    chk(lib.gpbdev_vecchia_get_sums(eng, sums.ctypes.data_as(C.POINTER(C.c_double))))
+    outputs["vecchia_nll_sums"] = sums[:3]  # y' Psi^-1 y, log|Psi|, #(D_i <= 0) of the last device-resident pass
     dev_ms = float(np.mean(kernel_ms))
     launches = lib.gpbdev_vecchia_launch_count(eng) - launches0  # factor + reduction kernel per step (L2-flush fills not counted)
     # ---- e2e timing through the C API with host buffers
@@ -435,6 +443,7 @@ def main():
         chk(lib.GPB_EvalNegLogLikelihood(mdl.handle, y_ptr, cp_ptr, None, C.byref(negll)))
     barrier()
     e2e_s = (time.perf_counter() - t0) / args.steps
+    outputs["negll_e2e"] = np.array([negll.value])
     # the same call with the response in ordinary (pageable) numpy memory — what a ctypes caller of the reference's package passes;
     # the engine stages it through its pinned buffer (dev_api.cu: gpbdev_vecchia_set_y)
     y_page = np.ascontiguousarray(y.copy())
@@ -447,6 +456,7 @@ def main():
         chk(lib.GPB_EvalNegLogLikelihood(mdl.handle, yp_ptr, cp_ptr, None, C.byref(negll)))
     barrier()
     e2e_page_s = (time.perf_counter() - t0) / args.steps
+    outputs["negll_e2e_pageable"] = np.array([negll.value])
     sampler.stop_flag = True; sampler.join(2)
 
     # max over ranks
@@ -555,6 +565,19 @@ def main():
                 line["cpu_baseline"] = {"value": v, "unit": "evals/s", "cores": ncores, "kind": "reference",
                                         "sample": "n=%d sub-problem of the same workload, 3 timed GPB_EvalNegLogLikelihood calls of the "
                                                   "unmodified reference CPU library; per-eval time scaled linearly to n=1e6" % ns}
+        if args.dump_outputs:
+            if laplace_res is not None:
+                outputs["laplace_negll"] = np.array([laplace_res["negll"]])
+            if gb is not None:
+                outputs["gpboost_cov_pars"] = np.array(gb["cov_pars"])
+            if dense_res is not None:
+                outputs["dense_negll"] = np.array([dense_res["negll"]])
+                outputs["dense_fit_cov_pars"] = np.array(dense_res["fit_cov_pars"])
+            if gg is not None:
+                outputs["gpboost_grouped_cov_pars"] = np.array(gg["grouped"]["cov_pars"])
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(arr, dtype=np.float64))
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

@@ -537,13 +537,19 @@ int gpbdev_vecchia_eval_async(gpbdev_vecchia_t h, int cov_type, double var, doub
   return launch_eval(h, cov_type, var, range, mode);
 }
 
-int gpbdev_vecchia_eval(gpbdev_vecchia_t h, int cov_type, double var, double range, int mode, double* out) {
-  if (!h || !out) return fail("gpbdev_vecchia_eval: null argument");
-  if (launch_eval(h, cov_type, var, range, mode)) return -1;
+int gpbdev_vecchia_get_sums(gpbdev_vecchia_t h, double* out) {
+  if (!h || !out) return fail("gpbdev_vecchia_get_sums: null argument");
+  CUDA_TRY(cudaSetDevice(h->device));
   CUDA_TRY(cudaMemcpyAsync(h->sums_host, h->sums, sizeof(double) * gpb::kNumAcc, cudaMemcpyDeviceToHost, h->stream));
   CUDA_TRY(cudaStreamSynchronize(h->stream));
   std::memcpy(out, h->sums_host, sizeof(double) * gpb::kNumAcc);
   return 0;
+}
+
+int gpbdev_vecchia_eval(gpbdev_vecchia_t h, int cov_type, double var, double range, int mode, double* out) {
+  if (!h || !out) return fail("gpbdev_vecchia_eval: null argument");
+  if (launch_eval(h, cov_type, var, range, mode)) return -1;
+  return gpbdev_vecchia_get_sums(h, out);
 }
 
 int gpbdev_vecchia_yaux(gpbdev_vecchia_t h, double* yaux_host) {

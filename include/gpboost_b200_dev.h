@@ -75,6 +75,8 @@ GPBDEV_EXPORT int gpbdev_vecchia_eval(gpbdev_vecchia_t h, int cov_type, double v
                                       double* out);
 /* same, asynchronous on the engine's stream and without the D2H of the sums (bench: device-only timing) */
 GPBDEV_EXPORT int gpbdev_vecchia_eval_async(gpbdev_vecchia_t h, int cov_type, double var, double range, int mode);
+/* the sums of the last evaluation (GPBDEV_NUM_SUMS doubles into a host buffer; waits for the engine's stream) */
+GPBDEV_EXPORT int gpbdev_vecchia_get_sums(gpbdev_vecchia_t h, double* out);
 
 /* After a STORE eval: y_aux = Psi^-1 y = B^T D^-1 B y (CalcYAux, re_model_template.h:9772) returned in
  * ORIGINAL observation order into a host buffer of n doubles. */

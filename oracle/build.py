@@ -7,6 +7,9 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _REPO = os.path.dirname(_HERE)
 _SRCS = ["vecchia_oracle.c", "tree_oracle.c"]
 _CXX_SRCS = ["shuffle_oracle.cpp"]
+# checkout of the unmodified reference: oracle/_ref is built from its sources and the drop-in tests take its Python package;
+# GPBOOST_REFERENCE names a checkout elsewhere
+REFERENCE_DIR = os.environ.get("GPBOOST_REFERENCE", "/root/reference")
 
 
 def oracle_lib_path():
@@ -45,9 +48,9 @@ def build_ref(jobs=8):
     out = ref_lib_path()
     if os.path.exists(out):
         return out
-    if not os.path.isdir("/root/reference/src"):
+    if not os.path.isdir(os.path.join(REFERENCE_DIR, "src")):
         return None
     subprocess.check_call(["make", "-f", os.path.join(_HERE, "Makefile.ref"), "-j%d" % jobs,
-                           "OUT=" + os.path.join(_HERE, "_ref")], cwd=_REPO,
+                           "REF=" + REFERENCE_DIR, "OUT=" + os.path.join(_HERE, "_ref")], cwd=_REPO,
                           stdout=subprocess.DEVNULL)
     return out

@@ -1,6 +1,6 @@
 """Staging of the UNMODIFIED reference Python package next to a chosen shared library (shared by the drop-in tests).
-The package is taken from /root/reference (build container) or from baseline/_ref/python-package (the copy __graft_entry__.build()
-places there — git-ignored, it travels to the GPU box like oracle/_ref); nothing of it is part of the product."""
+The package is taken from python-package/gpboost of the reference checkout oracle/_ref is built from (oracle.build.REFERENCE_DIR);
+nothing of it is part of this repository."""
 import json
 import os
 import subprocess
@@ -8,15 +8,12 @@ import sys
 import tempfile
 import textwrap
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = ["/root/reference/python-package/gpboost", os.path.join(ROOT, "baseline", "_ref", "python-package", "gpboost")]
+from oracle.build import REFERENCE_DIR
 
 
 def ref_package_dir():
-    for c in CANDIDATES:
-        if os.path.isdir(c):
-            return c
-    return None
+    pkg = os.path.join(REFERENCE_DIR, "python-package", "gpboost")
+    return pkg if os.path.isdir(pkg) else None
 
 
 def stage(lib_path):

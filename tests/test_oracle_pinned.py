@@ -1,6 +1,9 @@
 """The oracle (oracle/vecchia_oracle.c) is pinned against (1) the known-answer values hard-coded in the
 reference's own R tests, (2) golden vectors produced by the unmodified reference library
-(tests/golden/make_golden.py) and (3) — where oracle/_ref is present — live calls of that library."""
+(tests/golden/make_golden.py) and (3) the results of calls of that library on further cases (tests/golden/make_reference_golden.py)."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -9,6 +12,14 @@ from conftest import case_data
 from oracle import vecchia as ov
 
 CP = np.array([0.1, 1.6, 0.2])
+LIVE_CASES = (("matern", 1.5, 15, "random"), ("exponential", 0.5, 8, "none"), ("gaussian", 0., 10, "random"))
+LIVE_CP = np.array([0.4, 0.9, 0.12])
+
+
+@pytest.fixture(scope="module")
+def golden_ref():
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_golden.json")) as f:
+        return json.load(f)
 
 
 def test_r_known_answers_exact_gp():
@@ -50,17 +61,13 @@ def test_oracle_gradient_is_derivative_of_nll():
         assert abs(fd - g[k]) < 1e-5 * max(1., abs(g[k]))
 
 
-def test_oracle_matches_reference_library_live(ref_lib):
-    if ref_lib is None:
-        pytest.skip("oracle/_ref/lib_gpboost.so not built here")
-    from gpboost_b200 import GPModel
+def test_oracle_matches_reference_library_live(golden_ref):
     coords, y = datagen.synth(1200, 2, 21)
-    for cov, shape, m, ordering in (("matern", 1.5, 15, "random"), ("exponential", 0.5, 8, "none"), ("gaussian", 0., 10, "random")):
-        mdl = GPModel(gp_coords=coords, cov_function=cov, cov_fct_shape=shape, gp_approx="vecchia", num_neighbors=m,
-                      vecchia_ordering=ordering, seed=4, _lib=ref_lib)
-        o = ov.VecchiaOracle(coords, m, cov, shape, vecchia_ordering=ordering, seed=4)
-        cp = np.array([0.4, 0.9, 0.12])
-        a, b = mdl.neg_log_likelihood(cp, y), o.neg_log_likelihood(cp, y)
+    recs = golden_ref["vecchia_nll"]
+    assert [(r["cov_function"], r["cov_fct_shape"], r["num_neighbors"], r["vecchia_ordering"]) for r in recs] == list(LIVE_CASES)
+    for r in recs:
+        o = ov.VecchiaOracle(coords, r["num_neighbors"], r["cov_function"], r["cov_fct_shape"], vecchia_ordering=r["vecchia_ordering"], seed=4)
+        a, b = r["negll"], o.neg_log_likelihood(LIVE_CP, y)
         assert abs(a - b) <= 1e-10 * abs(a)
 
 

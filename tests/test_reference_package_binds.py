@@ -1,9 +1,9 @@
-"""Drop-in boundary, exercised with the UNMODIFIED reference Python package (python-package/gpboost of /root/reference, imported in
-place — nothing is copied): its module files are symlinked into a scratch directory next to lib_gpboost_b200.so under the name
-the package searches for (lib_gpboost.so, libpath.py:36). The package must import (every symbol it binds at load time resolves),
-build a Dataset through LGBM_DatasetCreateFromMat / SetField / GetField on the host, and reach the device-creating entries —
+"""Drop-in boundary, exercised with the UNMODIFIED reference Python package (python-package/gpboost of the reference checkout
+oracle/_ref is built from, imported in place — nothing is copied): its module files are symlinked into a scratch directory next to
+lib_gpboost_b200.so under the name the package searches for (lib_gpboost.so, libpath.py:36). The package must import (every symbol it
+binds at load time resolves), build a Dataset through LGBM_DatasetCreateFromMat / SetField / GetField on the host, and reach the device-creating entries —
 which, on this GPU-less container, must fail through the reference's own error channel (GPBoostError from LGBM_GetLastError)
-because the library has no CPU fallback. Skipped where /root/reference is absent (the GPU box)."""
+because the library has no CPU fallback. Skipped where there is no reference checkout."""
 import os
 import subprocess
 import sys
@@ -12,11 +12,13 @@ import textwrap
 
 import pytest
 
-REF_PKG = "/root/reference/python-package/gpboost"
+import dropin
+
+REF_PKG = dropin.ref_package_dir()
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_PKG), reason="reference sources not present")
+@pytest.mark.skipif(REF_PKG is None, reason="reference Python package not present (set GPBOOST_REFERENCE)")
 def test_unmodified_reference_package_loads_and_reaches_the_device_entries():
     lib = os.path.join(ROOT, "gpboost_b200", "lib_gpboost_b200.so")
     assert os.path.exists(lib)
@@ -59,7 +61,7 @@ def test_unmodified_reference_package_loads_and_reaches_the_device_entries():
     assert r.returncode == 0, r.stdout + r.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_PKG), reason="reference sources not present")
+@pytest.mark.skipif(REF_PKG is None, reason="reference Python package not present (set GPBOOST_REFERENCE)")
 def test_unmodified_reference_package_predicts_through_the_library(ref_lib):
     """gpb.Booster(model_str=...) / predict / save_model / Booster(model_file=...) of the unmodified package, bound to THIS library,
     on a model trained by the reference: predictions equal the reference library's own (host path, no device needed)."""

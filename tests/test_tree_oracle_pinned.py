@@ -1,5 +1,5 @@
 """Pins oracle/tree_oracle.c (+ the boosting restatement in oracle/tree.py) against trees grown by the unmodified
-reference library: the committed golden file (tests/golden/tree_golden.json) and, where oracle/_ref exists, a live run.
+reference library: the committed golden files (tests/golden/tree_golden.json, and a further run in tests/golden/reference_golden.json).
 Integer-valued features are used so that the reference's bins are known without restating its bin finder: value k sits
 in bin k (BinMapper::FindBin with <= max_bin distinct values; GreedyFindBin bin.cpp:83-98 puts bounds at midpoints)."""
 import json
@@ -12,11 +12,18 @@ import treedata
 from oracle import tree as ot
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+LIVE_SPEC = {"name": "live", "n": 3000, "F": 5, "kind": "int", "levels": 60, "num_leaves": 12, "min_data_in_leaf": 15, "num_iter": 2, "seed": 11}
 
 
 @pytest.fixture(scope="module")
 def tree_golden():
     with open(os.path.join(ROOT, "tests", "golden", "tree_golden.json")) as f:
+        return json.load(f)
+
+
+@pytest.fixture(scope="module")
+def golden_ref():
+    with open(os.path.join(ROOT, "tests", "golden", "reference_golden.json")) as f:
         return json.load(f)
 
 
@@ -49,18 +56,13 @@ def test_tree_oracle_matches_reference_golden(tree_golden):
         assert np.abs(score[:64] - np.array(rec["score_head"])).max() == 0.0
 
 
-def test_tree_oracle_matches_reference_live(ref_lib):
-    if ref_lib is None:
-        pytest.skip("oracle/_ref/lib_gpboost.so not built here")
-    from gpboost_b200.booster import Booster, Dataset, parse_model_string
-    spec = {"name": "live", "n": 3000, "F": 5, "kind": "int", "levels": 60, "num_leaves": 12, "min_data_in_leaf": 15, "num_iter": 2, "seed": 11}
+def test_tree_oracle_matches_reference_live(golden_ref):
+    from gpboost_b200.booster import parse_model_string
+    spec = LIVE_SPEC
     X, y, _ = treedata.make_case(spec)
-    params = treedata.booster_params(spec, reference=True)
-    b = Booster(params, Dataset(X, y, params=params, _lib=ref_lib), _lib=ref_lib)
-    for _ in range(spec["num_iter"]):
-        b.update()
-    g = parse_model_string(b.model_to_string())
+    rec = golden_ref["tree"]
+    g = parse_model_string(rec["model"])
     bins = np.ascontiguousarray(X.T.astype(np.uint8))
     trees, score, init = ot.boost_l2(bins, np.full(spec["F"], spec["levels"]), y, _cfg(spec), 0.1, spec["num_iter"])
     _check(trees, [{k: v for k, v in t.items()} for t in g], init, 1e-15)
-    assert np.abs(score - b.inner_predict_train()).max() == 0.0
+    assert np.abs(score - np.array(rec["score"])).max() == 0.0

@@ -1,9 +1,11 @@
 """GPU parity tests (run with -m gpu on the B200 box). Everything goes through the C ABI of
-lib_gpboost_b200.so; the oracle (and, where present, the unmodified reference library) is only the checker.
+lib_gpboost_b200.so; the oracle (and the stored results of the unmodified reference library) is only the checker.
 
 Tolerances: neighbour indices bit-exact; negative log-likelihood <= 1e-8 relative (north_star), in practice
 ~1e-13; B, D^-1, gradients and Psi^-1 y <= 1e-8 relative."""
 import ctypes as C
+import json
+import os
 
 import numpy as np
 import pytest
@@ -15,6 +17,8 @@ from oracle import vecchia as ov
 pytestmark = pytest.mark.gpu
 
 REL = 1e-8
+LIVE_KW = dict(cov_function="matern", cov_fct_shape=2.5, gp_approx="vecchia", num_neighbors=11, seed=6)
+LIVE_CP = np.array([0.2, 1.1, 0.3])
 
 
 def P(a, t=C.c_double):
@@ -25,6 +29,12 @@ def P(a, t=C.c_double):
 def lib(product_lib):
     assert product_lib.gpbdev_device_count() > 0, "no CUDA device visible — GPU tests need the B200 box"
     return product_lib
+
+
+@pytest.fixture(scope="module")
+def golden_ref():
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_golden.json")) as f:
+        return json.load(f)
 
 
 def chk(lib, rc):
@@ -181,18 +191,15 @@ def test_capi_response_gradient_matches_oracle(lib):
     assert np.abs(g - ya / s2).max() <= REL * np.abs(ya / s2).max()
 
 
-def test_capi_live_against_reference_library(lib, ref_lib):
-    if ref_lib is None:
-        pytest.skip("oracle/_ref/lib_gpboost.so not present")
+def test_capi_live_against_reference_library(lib, golden_ref):
     from gpboost_b200 import GPModel
     coords, y = datagen.synth(2500, 2, 29)
-    kw = dict(gp_coords=coords, cov_function="matern", cov_fct_shape=2.5, gp_approx="vecchia", num_neighbors=11, seed=6)
-    a, b = GPModel(**kw), GPModel(_lib=ref_lib, **kw)
-    cp = np.array([0.2, 1.1, 0.3])
-    va, vb = a.neg_log_likelihood(cp, y), b.neg_log_likelihood(cp, y)
+    a = GPModel(gp_coords=coords, **LIVE_KW)
+    rec = golden_ref["vecchia_capi"]
+    va, vb = a.neg_log_likelihood(LIVE_CP, y), rec["negll"]
     assert abs(va - vb) <= REL * abs(vb)
-    a.fit(y); b.fit(y)
-    assert abs(a.get_current_neg_log_likelihood() - b.get_current_neg_log_likelihood()) <= 1e-6 * abs(b.get_current_neg_log_likelihood())
+    a.fit(y)
+    assert abs(a.get_current_neg_log_likelihood() - rec["fit_negll"]) <= 1e-6 * abs(rec["fit_negll"])
 
 
 # ---------------------------------------------------------------------------------------- edge cases
